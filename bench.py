@@ -55,6 +55,7 @@ def parse():
     ap.add_argument("--weak", action="store_true", help="N > 1: one genome-equivalent of contigs per GPU instead of ONE genome sharded over the GPUs")
     ap.add_argument("--strong", action="store_true", help="(default for N > 1, kept for compatibility)")
     ap.add_argument("--extract-reads", type=int, default=0, help="config 5 extraction leg: alignment records in the CIGAR packet (0 = default)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="--impl b200: write the records of the last timed step to DIR/<name>.npy (see dump_outputs)")
     return ap.parse_args()
 
 
@@ -167,6 +168,39 @@ def run_reference(args):
         "e2e": {"value": value, "unit": UNIT, "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0},
     }
     print(json.dumps(line))
+
+
+DUMP_BUDGET_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, cands, genos, names):
+    """What a caller of the timed path receives (csv_fetch, or csv_fetch_gathered for N > 1) as float64 tables, one column
+    per record field in dtype order (int32 fields and the float64 QUAL convert exactly): cands.npy (_abi.CAND_DTYPE),
+    genos.npy (_abi.GENO_DTYPE), names.npy (supporting read ids) and counts.npy = [candidates, read ids].  The device
+    places each candidate's read-id slice wherever an atomic lands it, so the slices are written in candidate order and
+    names_off is rewritten to match.  Tables that together exceed 64 MB keep the same fraction of their rows, chosen by
+    a fixed seed, in order, so that two builds computing the same records write the same files."""
+    os.makedirs(out_dir, exist_ok=True)
+    off = cands["names_off"].astype(np.int64)
+    cnt = cands["names_cnt"].astype(np.int64)
+    new_off = np.cumsum(cnt) - cnt
+    names = names[np.repeat(off - new_off, cnt) + np.arange(int(cnt.sum()))]
+    cands = cands.copy()
+    cands["names_off"] = new_off
+
+    def table(a):
+        if a.dtype.names is None:
+            return a.astype(np.float64)
+        return np.concatenate([a[f].reshape(len(a), *(a.dtype[f].shape or (1,))) for f in a.dtype.names], axis=1).astype(np.float64)
+    tables = {"cands": table(cands), "genos": table(genos), "names": table(names)}
+    total = sum(t.nbytes for t in tables.values())
+    frac = min(1.0, (DUMP_BUDGET_BYTES - 4096) / max(total, 1))   # 4 KB for the .npy headers and counts.npy
+    for k, t in tables.items():
+        if frac < 1.0:
+            keep = int(len(t) * frac)
+            t = t[np.sort(np.random.default_rng(0).choice(len(t), keep, replace=False))]
+        np.save(os.path.join(out_dir, k + ".npy"), t)
+    np.save(os.path.join(out_dir, "counts.npy"), np.array([len(cands), len(names)], dtype=np.float64))
 
 
 def pinned_copy(torch, cols):
@@ -304,6 +338,8 @@ def main():
     dev_ms = e0.elapsed_time(e1)
     launches = eng.launch_count() - l0
     replays = eng.graph_replays() - g0
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, *(eng.fetch_gathered() if world > 1 else eng.fetch()))
     if world > 1:
         gathered = eng.gathered_counts()
     # noise bar: the same K steps timed once more, every step between its own events

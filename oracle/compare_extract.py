@@ -1,7 +1,16 @@
 """Compares extracted signature columns with the reference's candidate tuple lists (multisets)."""
 import collections
+import hashlib
 
 from cutesv_b200 import packing
+
+
+def digest_ins_seqs(cand):
+    """The candidate dict with every INS sequence (tuple field 3) replaced by a 64-bit SHA-256 prefix: keeps stored
+    goldens small while the comparison still covers the sequence content."""
+    out = dict(cand)
+    out["INS"] = [tuple(t[:3]) + ("sha256:" + hashlib.sha256(t[3].encode()).hexdigest()[:16],) + tuple(t[4:]) for t in cand["INS"]]
+    return out
 
 
 def tuples_from_columns(ex, chrom_names, read_names, query_of, cigar_of=None, merge=(10, 100)):

@@ -1,8 +1,8 @@
 """Runs the UNMODIFIED reference (/root/reference/src) on columnar inputs (TEST INFRASTRUCTURE).
 
-Only usable in the authoring container: /root/reference does not exist on the GPU box, so this
-module is imported by oracle/gen_golden.py (which commits its outputs under tests/golden/) and
-by tests that skip themselves when the reference is absent.
+Only usable where the reference sources are present, so this module is imported by the golden
+generators (oracle/gen_*.py), which commit the reference's outputs under tests/golden/; the tests
+compare against those files and never import the reference.
 
 pysam / cigar / Bio are not installed here; they are stubbed with the minimal surface the hot
 path touches (SURVEY.md section 8c).
@@ -167,6 +167,26 @@ def write_fake_bam(path, aln, chrom_names, lens, read_name):
         pickle.dump(dict(contigs=[(n, int(l)) for n, l in zip(chrom_names, lens)], reads=recs), f)
 
 
+def write_reference_workdir(tmp, tuples, n_pids=1):
+    """The reference's work dir under `tmp` (ends in "/"): per-worker signature pickles, then its rebuild
+    (process_process_sigs_type, cuteSV:750-857) into <TYPE>.pickle.  Returns sigs_index."""
+    main = modules()["main"]
+    os.mkdir(tmp + "signatures")
+    pids = list(range(100, 100 + n_pids))
+    for k in ("DEL", "INS", "DUP", "INV", "TRA", "reads"):
+        lst = tuples[k]
+        for j, pid in enumerate(pids):  # round-robin "tasks" over fake worker pids
+            with open("%ssignatures/%s%s.pickle" % (tmp, pid, k), "ab") as f:
+                pickle.dump(lst[j::n_pids], f)
+    sigs_index = {}
+    for k in ("DEL", "INS", "DUP", "INV", "TRA", "reads"):
+        r = main.process_process_sigs_type((k, tmp, pids, False))
+        sigs_index[r[0]] = r[1]
+        if r[0] == "reads":
+            sigs_index["reads_count"] = r[2]
+    return sigs_index
+
+
 def run_reference(sigs, reads, chrom_names, read_name, p, types_=("DEL", "INS", "INV", "DUP", "TRA"),
                   n_pids=1, tra_bam=None):
     """Reference rebuild (process_process_sigs_type, cuteSV:750-857) + clustering phase
@@ -175,24 +195,11 @@ def run_reference(sigs, reads, chrom_names, read_name, p, types_=("DEL", "INS", 
     TRA is run with action=False unless tra_bam (a fake-pysam BAM path) is given: its call_gt
     re-opens the BAM."""
     m = modules()
-    main = m["main"]
     tuples = to_tuples(sigs, reads, chrom_names, read_name)
     res = {}
     with tempfile.TemporaryDirectory() as d:
         tmp = d + "/"
-        os.mkdir(tmp + "signatures")
-        pids = list(range(100, 100 + n_pids))
-        for k in ("DEL", "INS", "DUP", "INV", "TRA", "reads"):
-            lst = tuples[k]
-            for j, pid in enumerate(pids):  # round-robin "tasks" over fake worker pids
-                with open("%ssignatures/%s%s.pickle" % (tmp, pid, k), "ab") as f:
-                    pickle.dump(lst[j::n_pids], f)
-        sigs_index = {}
-        for k in ("DEL", "INS", "DUP", "INV", "TRA", "reads"):
-            r = main.process_process_sigs_type((k, tmp, pids, False))
-            sigs_index[r[0]] = r[1]
-            if r[0] == "reads":
-                sigs_index["reads_count"] = r[2]
+        sigs_index = write_reference_workdir(tmp, tuples, n_pids)
         action = bool(p.genotype)
         if "DEL" in types_:
             for chr_ in sigs_index["DEL"]:

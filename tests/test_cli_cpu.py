@@ -1,24 +1,20 @@
 """CPU: CLI flag surface identical to the reference's parseArgs; task windows like cuteSV:1018-1044."""
-import pytest
+import json
+import os
 
+import golden_util
 from cutesv_b200 import cli
-from oracle import ref_harness
 
 
 def test_defaults_and_flags_match_reference():
-    if not ref_harness.available():
-        pytest.skip("reference not present (GPU box)")
-    ref_harness.modules()
-    from cuteSV.cuteSV_Description import parseArgs
-    for argv in (["a.bam", "r.fa", "o.vcf", "wd"],
-                 ["a.bam", "r.fa", "o.vcf", "wd", "--genotype", "-s", "3", "-l", "50", "-L", "-1", "-t", "4", "-b", "500", "-p", "-1", "-q", "10",
-                  "-r", "100", "-md", "500", "-mi", "500", "-sl", "20", "--max_cluster_bias_INS", "1000", "--diff_ratio_merging_INS", "0.9",
-                  "--max_cluster_bias_DEL", "1000", "--diff_ratio_merging_DEL", "0.5", "--max_cluster_bias_INV", "7", "--max_cluster_bias_DUP", "8",
-                  "--max_cluster_bias_TRA", "9", "--diff_ratio_filtering_TRA", "0.5", "--remain_reads_ratio", "0.7", "--report_readid",
-                  "--ignore_sequence", "--retain_work_dir", "--write_old_sigs", "-S", "HG002", "--gt_round", "100", "-include_bed", "x.bed"]):
-        a = vars(parseArgs(argv))
-        b = vars(cli.build_parser().parse_args(argv))
-        assert a == b
+    """The namespace the reference's parseArgs returned for the same argument lists (tests/golden/ref_cli_args.json,
+    oracle/gen_ref_golden.py)."""
+    cases = json.load(open(os.path.join(golden_util.GOLDEN, "ref_cli_args.json")))
+    assert len(cases) == 2
+    for case in cases:
+        got = vars(cli.build_parser().parse_args(case["argv"]))
+        assert got == case["args"]
+        assert {k: type(v) for k, v in got.items()} == {k: type(v) for k, v in case["args"].items()}
 
 
 def test_task_windows_float_bounds():

@@ -1,6 +1,10 @@
 """CPU: the drop-in resolution_* entry points (work-dir pickles -> columns -> one cluster call -> the reference's rows)
 with the kernels replaced by the pipeline emulator, against the rows the REAL reference produced (tests/golden).
 The -m gpu twin is tests/test_gpu_dropin.py."""
+import hashlib
+import json
+import os
+
 import pytest
 
 import golden_util
@@ -77,30 +81,16 @@ def test_dropins_batch_one_cluster_call_per_type(tmp_path):
 
 @pytest.mark.parametrize("name", ["cfg2_s0p002", "adv034"])
 def test_reference_reads_a_repo_written_work_dir(tmp_path, name):
-    """--retain_work_dir compatibility the other way round: the REAL reference's run_del / run_ins / run_inv / run_dup
-    (unmodified, imported from /root/reference) over <TYPE>.pickle + sigindex written by cutesv_b200.workdir give the rows
-    of the golden (which the reference produced from its own work dir)."""
-    from oracle import ref_harness
-    if not ref_harness.available():
-        pytest.skip("reference not present (GPU box)")
-    m = ref_harness.modules()
+    """--retain_work_dir compatibility the other way round: <TYPE>.pickle + sigindex written by cutesv_b200.workdir are
+    byte for byte the work dir the REAL reference's own rebuild writes from the same signatures (tests/golden/ref_workdir.json,
+    oracle/gen_ref_golden.py), from which the reference produced the golden rows; so its run_del / run_ins / run_inv /
+    run_dup read the same lists at the same offsets."""
+    want = json.load(open(os.path.join(golden_util.GOLDEN, "ref_workdir.json")))[name]
     case = golden_util.load_case(name)
-    p = case["params"]
     path = str(tmp_path) + "/"
     idx = workdir.write_workdir(path, _tuples(case))
-    action = bool(p.genotype)
-    got = {}
-    for chrom in idx["DEL"]:
-        got[("DEL", chrom)] = m["indel"].run_del((path, chrom, "DEL", p.min_support, p.ratio_del, p.bias_del, p.min_support_allele, "", action,
-                                                  p.gt_round, p.remain_reads_ratio, idx))[1]
-    for chrom in idx["INS"]:
-        got[("INS", chrom)] = m["indel"].run_ins((path, chrom, "INS", p.min_support, p.ratio_ins, p.bias_ins, p.min_support_allele, "", action,
-                                                  p.gt_round, p.remain_reads_ratio, idx))[1]
-    for chrom in idx["INV"]:
-        got[("INV", chrom)] = m["inv"].run_inv((path, chrom, "INV", p.min_support, p.bias_inv, p.min_size, "", action, p.max_size, p.gt_round, idx))[1]
-    for chrom in idx["DUP"]:
-        got[("DUP", chrom)] = m["dup"].run_dup((path, chrom, p.min_support, p.bias_dup, p.min_size, "", action, p.max_size, p.gt_round, idx))[1]
-    got = {k: v for k, v in got.items() if v}
-    want = {k: v for k, v in case["rows"].items() if k[0] != "TRA"}
-    d = compare.diff_rows(want, got)
-    assert not d and sum(len(v) for v in got.values()) > 0, "\n".join(d[:4])
+    assert json.loads(json.dumps(idx)) == want["sigs_index"]
+    assert sum(idx["reads_count"].values()) > 0 and any(idx[t] for t in ("DEL", "INS", "INV", "DUP"))
+    for t, digest in want["sha256"].items():
+        with open("%s%s.pickle" % (path, t), "rb") as f:
+            assert hashlib.sha256(f.read()).hexdigest() == digest, t

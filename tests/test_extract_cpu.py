@@ -1,15 +1,16 @@
 """CPU: the extraction logic (cutesv_b200/csrc/extract_core.h through the emulator) against golden
-tuples produced by the REAL reference's parse_read, and against the reference itself when present."""
+tuples produced by the REAL reference's parse_read."""
+import functools
+import gzip
 import json
 import os
 
-import numpy as np
 import pytest
 
 import emul_lib
 import golden_util
 from cutesv_b200 import _abi, packing, synth
-from oracle import compare_extract, ref_harness
+from oracle import compare_extract
 
 
 EXTRACT_GOLDENS = ["extract_s0", "extract_s1", "extract_s2", "extract_s3", "extract_s4", "extract_s5", "extract_s6",
@@ -43,17 +44,22 @@ def test_emulator_matches_reference_golden(name):
     assert not compare_extract.diff_extract(ref_c, ref_r, gc, gr)
 
 
-@pytest.mark.skipif(not ref_harness.available(), reason="reference not present (GPU box)")
+@functools.lru_cache(maxsize=None)
+def _live_goldens():
+    with gzip.open(os.path.join(golden_util.GOLDEN, "extract_live.json.gz"), "rt") as f:
+        return json.load(f)
+
+
 @pytest.mark.parametrize("seed", range(500, 520))
 def test_emulator_matches_live_reference(seed):
-    rng = np.random.default_rng(seed)
-    p = _abi.default_params(min_size=int(rng.choice([30, 50, 10])), max_size=int(rng.choice([-1, 100000, 2000])),
-                            min_mapq=int(rng.choice([20, 0, 30])), max_split_parts=int(rng.choice([7, -1, 2, 3])),
-                            min_read_len=int(rng.choice([500, 100])), min_siglength=int(rng.choice([10, 30])),
-                            merge_del_threshold=int(rng.choice([0, 500])), merge_ins_threshold=int(rng.choice([100, 500, 0])))
-    reads, (gc, gr), _ = _run(seed, 120, p)
-    ref_c, ref_r = ref_harness.run_parse_reads(reads, p)
-    assert not compare_extract.diff_extract(ref_c, ref_r, gc, gr)
+    """A random flag setting per seed: the reference's parse_read output on the same packet, INS sequences compared by
+    digest (tests/golden/extract_live.json.gz, oracle/gen_ref_golden.py)."""
+    meta = _live_goldens()[str(seed)]
+    p = _abi.default_params(**meta["params"])
+    reads, (gc, gr), _ = _run(seed, meta["n_reads"], p)
+    ref_c = {k: [tuple(t) for t in v] for k, v in meta["candidate"].items()}
+    ref_r = [tuple(t) for t in meta["rows"]]
+    assert not compare_extract.diff_extract(ref_c, ref_r, compare_extract.digest_ins_seqs(gc), gr)
 
 
 def test_acquire_clip_pos():

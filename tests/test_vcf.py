@@ -52,18 +52,10 @@ def test_header_shape():
 
 
 def test_header_matches_reference_when_present():
-    from oracle import ref_harness
-    if not ref_harness.available():
-        pytest.skip("reference not present (GPU box)")
-    import io
-    ref_harness.modules()
-    from cuteSV.cuteSV_Description import Generation_VCF_header
-    buf = io.StringIO()
-    contigs = [["1", 1000], ["X", 77]]
-    argv = ["a.bam", "r.fa", "o.vcf", "w", "--genotype"]
-    Generation_VCF_header(buf, contigs, "NULL", argv)
-    ref = buf.getvalue().splitlines()
-    got = vcf.header_lines(contigs, "NULL", argv)[:-1]
+    """Header lines the reference's Generation_VCF_header wrote (tests/golden/ref_vcf_header.json, oracle/gen_ref_golden.py)."""
+    case = json.load(open(os.path.join(golden_util.GOLDEN, "ref_vcf_header.json")))
+    ref = case["lines"]
+    got = vcf.header_lines(case["contigs"], case["sample"], case["argv"])[:-1]
     assert len(ref) == len(got)
     for a, b in zip(ref, got):
         if a.startswith("##fileDate"):
